@@ -25,6 +25,14 @@ extraction: images H2D + embeddings D2H per step (FeatureExtractor.extract_cbir)
 `roofline` times the dominant kernel alone with CUDA events (tensor bound, peaks from MEASURED_PEAKS.json; `traffic` = DRAM bytes
 per launch from the ncu captures under profiles/).  `cpu_baseline` is the oracle's port of the reference CPU formulation on the
 host cores (thread count calibrated, samples bounded); `--impl reference` prints the same line for that CPU port alone.
+
+`--dump-outputs DIR` writes what the last timed step of each leg returned to its caller, as DIR/<name>.npy (float32; ids as
+float64): train_loss, train_vit_loss, extract_embeddings, extract_vit_embeddings, extract_vitl_embeddings, retrieval_scores,
+retrieval_ids.  Inputs and weights are seeded, so two builds run with the same arguments can be compared file by file.  Above
+64 MB in all, every array keeps the same fixed, seeded sample of its rows.  bench.py writes nothing else to disk.
+Embeddings, scores and ids repeat bit for bit from run to run.  The train losses do not: the weight-gradient reductions add
+with float atomics, and after the default 3 warm-up + 20 timed steps two runs differ by up to about 1e-2 relative (6e-3 seen
+for train_vit_loss over three runs on one B200, 1000 W power limit).
 """
 from __future__ import annotations
 
@@ -58,6 +66,8 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle parity check of the retrieval leg")
     ap.add_argument("--train-batch", type=int, default=128)
     ap.add_argument("--only", default="all", choices=["all", "both", "train", "extract", "retrieval"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each leg returned as DIR/<name>.npy (at most 64 MB in all)")
     return ap.parse_args()
 
 
@@ -313,16 +323,18 @@ class Ctx:
 
 
 def timed(ctx, fn, steps, warmup):
-    """W warm-up calls, then K calls bracketed by barrier + synchronize; CUDA events; max over ranks."""
+    """W warm-up calls, then K calls bracketed by barrier + synchronize; CUDA events; max over ranks.
+    Returns the ms per call and what the last call returned."""
     import torch
     import torch.distributed as dist
     for _ in range(max(3, warmup)):
         fn()
     ctx.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    out = None
     e0.record()
     for _ in range(steps):
-        fn()
+        out = fn()
     e1.record()
     ctx.barrier()
     ms = e0.elapsed_time(e1)
@@ -330,7 +342,35 @@ def timed(ctx, fn, steps, warmup):
         t = torch.tensor([ms], device=ctx.dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
-    return ms / steps
+    return ms / steps, out
+
+
+MAX_DUMP_BYTES = 60 * 10**6  # array data; with the .npy headers the files stay under 64 MB however it is counted
+
+
+def keep_outputs(ctx, args, **tensors):
+    """--dump-outputs: host copies of what a leg's last timed step returned, taken right after its timed loop (the untimed
+    calls that follow may reuse the same buffers)."""
+    if args.dump_outputs:
+        ctx.outputs.update({name: t.detach().cpu() for name, t in tensors.items()})
+
+
+def dump_outputs(outputs, out_dir):
+    """DIR/<name>.npy in float32 (float64 kept; integers as float64, exact below 2**53).  Above MAX_DUMP_BYTES in all, every
+    array keeps the same fraction of its rows, chosen by a fixed seed, so a given set of arguments always dumps the same rows."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for name, t in outputs.items():
+        dt = torch.float64 if t.dtype == torch.float64 or not t.is_floating_point() else torch.float32
+        arrays[name] = t.to(dt).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > MAX_DUMP_BYTES and a.ndim > 0:
+            keep = max(1, a.shape[0] * MAX_DUMP_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def peak_tflops():
@@ -428,7 +468,8 @@ def bench_extract(ctx, args):
         state["i"] += 1
         return model.embed(x, l2_normalize=True)
 
-    ms = timed(ctx, step_dev, args.steps, args.warmup)
+    ms, emb = timed(ctx, step_dev, args.steps, args.warmup)
+    keep_outputs(ctx, args, extract_embeddings=emb)
     value = ctx.world * B / (ms * 1e-3)
 
     # e2e: the reference-facing call FeatureExtractor.extract_cbir(dataloader, device) -> numpy, fed from pinned host
@@ -468,7 +509,7 @@ def bench_extract(ctx, args):
             "h2d": B * 3 * IMG * IMG * 4, "d2h": B * FEAT * 4, "batch": B}
 
 
-def bench_extract_vit(ctx, args, name="vit_base_patch16_224", img=IMG, batch=None, title="ViT-B/16"):
+def bench_extract_vit(ctx, args, name="vit_base_patch16_224", img=IMG, batch=None, title="ViT-B/16", leg="extract_vit"):
     """Secondary row (BASELINE config 5 family): CBIR extraction with a Transformer backbone, ViT-B/16 224^2, random-init
     weights, batch = --batch per GPU.  Device-resident and end-to-end (FeatureExtractor.extract_cbir from pinned host batches)."""
     import torch
@@ -487,7 +528,8 @@ def bench_extract_vit(ctx, args, name="vit_base_patch16_224", img=IMG, batch=Non
         state["i"] += 1
         return model.embed(x, l2_normalize=True)
 
-    ms = timed(ctx, step_dev, args.steps, args.warmup)
+    ms, emb = timed(ctx, step_dev, args.steps, args.warmup)
+    keep_outputs(ctx, args, **{f"{leg}_embeddings": emb})
     host_x = [torch.randn(B, 3, IMG_, IMG_).pin_memory() for _ in range(2)]
     extractor = FeatureExtractor(model)
 
@@ -552,7 +594,8 @@ def bench_train(ctx, args):
         state["i"] += 1
         return trainer.step(pool[i], labels[i])
 
-    ms = timed(ctx, step_dev, args.steps, args.warmup)
+    ms, loss = timed(ctx, step_dev, args.steps, args.warmup)
+    keep_outputs(ctx, args, train_loss=loss)
     value = ctx.world * B / (ms * 1e-3)
 
     host_x = [torch.randn(B, 3, IMG, IMG).pin_memory() for _ in range(2)]
@@ -569,7 +612,7 @@ def bench_train(ctx, args):
         loss = trainer.step(x, y)
         return loss.item()
 
-    e2e_ms = timed(ctx, step_e2e, args.steps, args.warmup)
+    e2e_ms, _ = timed(ctx, step_e2e, args.steps, args.warmup)
     peak_s = 1422.7
     try:
         peak_s = float(json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["bf16_tflops_sustained"])
@@ -611,7 +654,8 @@ def bench_train_vit(ctx, args):
         state["i"] += 1
         return trainer.step(pool[i], labels[i])
 
-    ms = timed(ctx, step_dev, args.steps, args.warmup)
+    ms, loss = timed(ctx, step_dev, args.steps, args.warmup)
+    keep_outputs(ctx, args, train_vit_loss=loss)
     host_x = [torch.randn(B, 3, IMG, IMG).pin_memory() for _ in range(2)]
     host_y = [torch.randint(0, 1000, (B,)).pin_memory() for _ in range(2)]
     n_e2e = max(3, args.warmup) + args.steps
@@ -621,7 +665,7 @@ def bench_train_vit(ctx, args):
         x, y = next(feed)
         return trainer.step(x, y).item()
 
-    e2e_ms = timed(ctx, step_e2e, args.steps, args.warmup)
+    e2e_ms, _ = timed(ctx, step_e2e, args.steps, args.warmup)
     gflop = 3 * 35.28
     peak_s = 1422.7
     try:
@@ -674,8 +718,9 @@ def bench_retrieval(ctx, args):
     def step_dev():  # device-resident: no host synchronisation inside a search; overflow is checked once after the timed loop
         return sharded_flat_search(index, q_local, q_sizes, k, defer_check=True)
 
-    ms = timed(ctx, step_dev, args.steps, args.warmup)
+    ms, (s_last, i_last) = timed(ctx, step_dev, args.steps, args.warmup)
     index.check_status(all_ranks=True)  # raises on every rank if any shard overflowed its candidate lists during the loop
+    keep_outputs(ctx, args, retrieval_scores=s_last, retrieval_ids=i_last)
     value = nq * ng / (ms * 1e-3)
 
     # parity check, outside the timed region: 64 sampled query rows of THIS search (single GPU or sharded) against the
@@ -714,7 +759,7 @@ def bench_retrieval(ctx, args):
             i_host.copy_(i, non_blocking=True)
         torch.cuda.synchronize()
 
-    e2e_ms = timed(ctx, step_e2e, args.steps, args.warmup)
+    e2e_ms, _ = timed(ctx, step_e2e, args.steps, args.warmup)
 
     roof = None
     ngl = hi - lo
@@ -765,9 +810,10 @@ def main():
 
     import torch
     import torch.distributed as dist
-    from visiondk_b200 import _lib, build
+    from visiondk_b200 import _lib
 
     ctx = Ctx()
+    ctx.outputs = {}
     ctx.world = int(os.environ.get("WORLD_SIZE", "1"))
     ctx.rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -777,8 +823,7 @@ def main():
     ctx.dev = torch.device("cuda", local_rank)
     if ctx.world > 1:
         dist.init_process_group("nccl", device_id=ctx.dev)
-    build.build()
-    _lib.load()
+    _lib.load()  # the library build() left in the tree; bench.py compiles nothing, so the tree may be read-only
     _lib.require_device()
 
     def barrier():
@@ -802,10 +847,12 @@ def main():
     torch.cuda.empty_cache()
     # BASELINE configs[4]: the CLIP ViT-L/14 tower at 336^2 (timm vit_large_patch14_clip_336: 577 tokens, width 1024, 24 blocks)
     exl = bench_extract_vit(ctx, args, name="vit_large_patch14_clip_336", img=336, batch=max(8, args.batch // 4),
-                            title="ViT-L/14 (CLIP tower)") if want("extract") else None
+                            title="ViT-L/14 (CLIP tower)", leg="extract_vitl") if want("extract") else None
     torch.cuda.empty_cache()
     rt = bench_retrieval(ctx, args) if want("retrieval") else None
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(ctx.outputs, args.dump_outputs)
 
     cpu = {}
     if ctx.rank == 0 and ctx.world == 1 and not args.no_cpu_baseline and (ex is not None or tr is not None):

@@ -1,4 +1,4 @@
-"""Generates tests/golden/*.npz by executing the REFERENCE's own modules (authoring container only).
+"""Generates tests/golden/*.npz by executing the REFERENCE's own modules, and copies its two faceX configs there as fixtures.
 
     python oracle/make_golden.py            # needs /root/reference; never runs on the GPU box
 
@@ -269,6 +269,15 @@ def preprocess():
     np.savez_compressed(os.path.join(OUT, "preprocess_ref.npz"), **out)
 
 
+def configs():
+    """The reference's own configs/faceX/{cbir,face}.yaml, byte for byte: tests/test_config_surface_cpu.py parses them through
+    engine.vision_engine.yaml_load + check, tests/test_cbir_folder_cpu.py reads their val augment list."""
+    import shutil
+    os.makedirs(os.path.join(OUT, "ref_configs"), exist_ok=True)
+    for name in ("cbir.yaml", "face.yaml"):
+        shutil.copyfile(os.path.join(REF, "configs", "faceX", name), os.path.join(OUT, "ref_configs", name))
+
+
 def ema_sgd_sched():
     ema_mod = load("models/ema.py", "ref_ema")
     sched = load("engine/scheduler.py", "ref_sched")
@@ -310,4 +319,5 @@ if __name__ == "__main__":
     ema_sgd_sched()
     neck()
     preprocess()
+    configs()
     print("golden vectors written to", OUT)

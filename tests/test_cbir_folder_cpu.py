@@ -110,12 +110,11 @@ def test_val_augment_parsing():
 
 
 def test_reference_cbir_yaml_val_list_is_the_supported_one():
-    """The val augment list of the reference's own configs/faceX/cbir.yaml (copied into tests by value: the reference tree is not
-    on the GPU box) parses to its image size and the ImageNet statistics."""
+    """The val augment list of the reference's own configs/faceX/cbir.yaml (written out by value, and checked against the
+    file's fixture copy tests/golden/ref_configs/cbir.yaml) parses to its image size and the ImageNet statistics."""
     ref_list = [{"resize_and_padding": {"size": 224, "training": False}}, {"to_tensor": "no_params"},
                 {"normalize": {"mean": [0.485, 0.456, 0.406], "std": [0.229, 0.224, 0.225]}}]
     assert parse_val_augment(ref_list) == (224, (0.485, 0.456, 0.406), (0.229, 0.224, 0.225))
-    if os.path.isdir("/root/reference"):  # authoring container: check the copy against the file itself
-        import yaml
-        with open("/root/reference/configs/faceX/cbir.yaml") as f:
-            assert yaml.safe_load(f)["data"]["val"]["augment"] == ref_list
+    import yaml
+    with open(os.path.join(os.path.dirname(__file__), "golden", "ref_configs", "cbir.yaml")) as f:
+        assert yaml.safe_load(f)["data"]["val"]["augment"] == ref_list

@@ -1,8 +1,8 @@
 """The configs/*.yaml surface (SURVEY.md §5, north_star "keeping the ... configs/*.yaml surface"): the reference's own
 configs/faceX/{face,cbir}.yaml parse unchanged through engine.vision_engine.yaml_load and satisfy engine.vision_engine.check's
 schema (utils/checks.py:225-229) once `data.root` points at data that exists here; the class-count assert (checks.py:111-143) fires
-like the reference's.  The reference files are read from /root/reference when present (authoring container); the repo's own
-config is always checked."""
+like the reference's.  The reference files are byte-for-byte copies kept as fixtures (tests/golden/ref_configs/,
+oracle/make_golden.py::configs)."""
 import copy
 import os
 
@@ -11,8 +11,8 @@ import pytest
 from engine.vision_engine import check, yaml_load
 from visiondk_b200.backbone import BackboneFactory
 
-REF = "/root/reference/configs/faceX"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = os.path.join(ROOT, "tests", "golden", "ref_configs")
 
 
 def test_own_config_passes_the_checks():
@@ -30,7 +30,6 @@ def test_own_config_passes_the_checks():
         check("classification", cfgs)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted (GPU box)")
 @pytest.mark.parametrize("name,task", [("cbir.yaml", "cbir"), ("face.yaml", "face")])
 def test_reference_yaml_parses_unchanged_and_passes_the_schema(name, task):
     cfgs = yaml_load(os.path.join(REF, name))

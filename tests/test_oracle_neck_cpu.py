@@ -23,8 +23,19 @@ def build(tag, z):
     return m
 
 
+@pytest.fixture
+def golden_threads():
+    """neck_ref.npz was minted with 8 intra-op CPU threads.  The CPU kernels split their reductions by thread count, and the
+    train-mode gradients of the 6-image batch are ill-conditioned: at any other count the Transformer neck's Linear weight
+    gradient moves by up to 3e-4 (float64 misses the golden by as much).  The test runs with the golden's 8 threads."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.mark.parametrize("tag", ["cnn", "vit"])
-def test_oracle_wrapper_reproduces_the_reference_wrapper(tag):
+def test_oracle_wrapper_reproduces_the_reference_wrapper(tag, golden_threads):
     z = np.load(GOLD)
     m = build(tag, z)
     sd = m.state_dict()

@@ -8,13 +8,11 @@ import os
 import numpy as np
 import pytest
 
-from conftest import not_yet_run_on_gpu
 from visiondk_b200.preprocess import resize_pad_normalize
 
 pytestmark = pytest.mark.gpu
 
 
-@not_yet_run_on_gpu
 def test_device_pipeline_reproduces_the_reference_tensors(lib):
     z = np.load(os.path.join(os.path.dirname(__file__), "golden", "preprocess_ref.npz"))
     mean, std = tuple(float(v) for v in z["mean"]), tuple(float(v) for v in z["std"])

@@ -7,7 +7,6 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import not_yet_run_on_gpu
 from oracle import preprocess as P
 
 pytestmark = pytest.mark.gpu
@@ -32,14 +31,14 @@ def make_tree(root, n_ids=6, per_gallery=4, per_query=2):
                 Image.fromarray(img).save(os.path.join(d, f"img_{j}.png"))
 
 
-@not_yet_run_on_gpu
 def test_valuate_on_an_image_folder(lib, tmp_path):
     from engine.cbir.evaluation import compute_metrics, valuate
     from engine.cbir.folder import CBIRFolderData, read_image
     from visiondk_b200.backbone import TimmWrapper
     from visiondk_b200.retrieval import FlatIPIndex
     make_tree(str(tmp_path))
-    model = TimmWrapper("toy", 32, SIZE, pretrained=False, depths=(1, 1, 1, 1), dims=(64, 64, 128, 128)).cuda().eval()
+    # 64-d embeddings: the top-k search takes widths that are multiples of 64 (vdk_topk_plan_default)
+    model = TimmWrapper("toy", 64, SIZE, pretrained=False, depths=(1, 1, 1, 1), dims=(64, 64, 128, 128)).cuda().eval()
     metrics_cfg = {"metrics": ["mrr", "recall", "precision", "auc", "ndcg"], "cutoffs": [1, 3, 5]}
     data_cfg = {"root": str(tmp_path), "nw": 2, "val": {"bs": 5, "augment": AUGMENT, "metrics": metrics_cfg}}
     got = valuate(model, data_cfg, "cuda", image_size=SIZE)
@@ -56,7 +55,7 @@ def test_valuate_on_an_image_folder(lib, tmp_path):
             out.append(model.embed(torch.from_numpy(x).cuda(), l2_normalize=True))
         return torch.cat(out)
 
-    index = FlatIPIndex(32, "cuda")
+    index = FlatIPIndex(64, "cuda")
     index.add(embed(data.gallery_files))
     scores, ids = index.search_device(embed(data.query_files), 5, resolve_overflow=True)
     want = compute_metrics(ids, scores, data.query_labels(), data.gallery_labels(), metrics=metrics_cfg["metrics"],
@@ -70,7 +69,6 @@ def test_valuate_on_an_image_folder(lib, tmp_path):
     assert results == [[data.gallery_files[j] for j in row] for row in ids.cpu().tolist()]
 
 
-@not_yet_run_on_gpu
 def test_extract_face_names_and_features(lib):
     """FeatureExtractor.extract_face (models/faceX/face_model.py:93-118): keys "<parent dir>/<file>", values = the rows
     extract_cbir_device returns for the same tensors."""
@@ -89,7 +87,6 @@ def test_extract_face_names_and_features(lib):
     assert ext.extract_face([], "cuda") == {}
 
 
-@not_yet_run_on_gpu
 def test_face_task_pair_verification(lib, tmp_path):
     """engine/faceX/evaluation.py::valuate: (a) synthetic:// root -> a (mean, std) in range that beats chance on the
     identity-structured images; (b) a pair file over <root>/val/ images == the same protocol assembled by hand."""
