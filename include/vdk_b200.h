@@ -296,7 +296,8 @@ int vdk_vit_pack(const vdk_vit_tensors* params, vdk_vit_net* net, void* stream);
 size_t vdk_vit_train_workspace_bytes(const vdk_vit_net* net, int batch);
 /* Train-mode forward of TimmWrapper('vit_*') (timm_wrapper.py:51-54; neck :42-47 with BatchNorm1d batch statistics,
  * running stats updated): images fp32 NCHW -> out_feats fp32 [batch, feat_dim]; activations saved in `workspace`.
- * Needs 3*patch*patch % 8 == 0 and at most 208 tokens (the attention backward keeps one head's P in shared memory). */
+ * Needs 3*patch*patch % 8 == 0; any token count (the attention backward runs the mma.sync kernel up to 208 tokens, the tcgen05
+ * pair of vdk_attention_bwd_tc beyond). */
 int vdk_vit_train_forward(const vdk_vit_net* net, const vdk_vit_tensors* params, const float* images, int batch, float bn_momentum,
                           float* out_feats, void* workspace, size_t workspace_bytes, void* stream);
 /* d_feats fp32 [batch, feat_dim] -> gradients ACCUMULATED (+=) into `grads`. */
@@ -313,6 +314,14 @@ int vdk_vit_train_backward_range(const vdk_vit_net* net, const vdk_vit_tensors* 
 int vdk_attention_fwd_lse(const void* qkv, int batch, int tokens, int heads, int head_dim, void* out, float* lse2, void* stream);
 int vdk_attention_bwd(const void* qkv, const void* out, const void* d_out, const float* lse2, int batch, int tokens, int heads,
                       int head_dim, void* dqkv, void* stream);
+/* The same backward on tcgen05 for any token count (the mma.sync kernel above keeps one head's P in shared memory and stops at
+ * 208 tokens).  Replaces timm's Attention backward inside `scaler.scale(loss).backward()` (engine/procedure/train.py:206) for long
+ * sequences (ViT-B/8 at 224^2: 785 tokens, ViT-B/16 at 384^2: 577).  Two kernels on `stream`; no atomics, so dqkv is the same bits on every run.
+ * workspace: caller-owned device memory of at least vdk_attention_bwd_tc_workspace_bytes(...) bytes, 16-byte aligned (holds
+ * D = rowsum(d_out * out) per (image, head, token)).  head_dim must be 64.  Host-only sizing: returns 0 for a bad shape. */
+size_t vdk_attention_bwd_tc_workspace_bytes(int batch, int tokens, int heads, int head_dim);
+int vdk_attention_bwd_tc(const void* qkv, const void* out, const void* d_out, const float* lse2, int batch, int tokens, int heads,
+                         int head_dim, void* dqkv, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- margin-softmax heads + cross-entropy --------------------------------------------------- */
 /* Replaces ArcFace.forward (models/faceX/head/arcface.py:20-36), CircleLoss.forward (models/faceX/head/

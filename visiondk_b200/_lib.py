@@ -99,6 +99,8 @@ SIGNATURES = {
     "vdk_vit_train_backward_range": (_i, [_p, _p, _p, _p, _i, _p, _sz, _p, _i, _i]),
     "vdk_attention_fwd_lse": (_i, [_p, _i, _i, _i, _i, _p, _p, _p]),
     "vdk_attention_bwd": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p, _p]),
+    "vdk_attention_bwd_tc_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "vdk_attention_bwd_tc": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _sz, _p]),
     "vdk_vit_forward": (_i, [_p, _p, _i, _i, _p, _p, _sz, _p]),
     "vdk_attention_fwd": (_i, [_p, _i, _i, _i, _i, _p, _p]),
     "vdk_convnext_workspace_bytes": (_sz, [_p, _i]),

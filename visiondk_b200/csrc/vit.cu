@@ -544,6 +544,22 @@ static int launch_attention_bwd(const __nv_bfloat16* qkv, const __nv_bfloat16* o
   return VDK_OK;
 }
 
+size_t attention_bwd_tc_workspace_bytes(int B, int N, int H);  // attention_bwd_tc.cu
+int launch_attention_bwd_tc(const __nv_bfloat16* qkv, const __nv_bfloat16* out, const __nv_bfloat16* d_out, const float* lse2, int B,
+                            int N, int H, __nv_bfloat16* dqkv, void* workspace, size_t workspace_bytes, cudaStream_t s);
+
+// The tcgen05 pair (attention_bwd_tc.cu) for any token count: kernel Q writes D_i = sum_d dO_id O_id into the workspace and dQ,
+// kernel KV reads D and writes dK, dV.  It executes 14 N^2 64 flops per (image, head) (no atomics: dS is recomputed on the key side);
+// the profile keeps the algorithmic 10 N^2 64 of the mma.sync kernel, so both report the same rate for the same time.
+static int launch_attention_bwd_pair(const __nv_bfloat16* qkv, const __nv_bfloat16* o, const __nv_bfloat16* d_o, const float* lse2,
+                                     int B, int N, int H, int head_dim, __nv_bfloat16* dqkv, void* workspace, size_t workspace_bytes,
+                                     cudaStream_t s) {
+  ProfScope prof(kProfAttention, 10.0 * static_cast<double>(B) * H * N * N * 64.0,
+                 2.0 * static_cast<double>(B) * N * H * 64.0 * 8.0, s);
+  VDK_REQUIRE(head_dim == kAttD, "attention backward: head_dim must be 64 (got %d)", head_dim);
+  return launch_attention_bwd_tc(qkv, o, d_o, lse2, B, N, H, dqkv, workspace, workspace_bytes, s);
+}
+
 static size_t up256v(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
 
 struct VitLayout {
@@ -607,6 +623,19 @@ extern "C" int vdk_attention_bwd(const void* qkv, const void* out, const void* d
   return launch_attention_bwd(reinterpret_cast<const __nv_bfloat16*>(qkv), reinterpret_cast<const __nv_bfloat16*>(out),
                               reinterpret_cast<const __nv_bfloat16*>(d_out), lse2, batch, tokens, heads, head_dim,
                               reinterpret_cast<__nv_bfloat16*>(dqkv), reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" size_t vdk_attention_bwd_tc_workspace_bytes(int batch, int tokens, int heads, int head_dim) {
+  if (head_dim != kAttD) return 0;
+  return attention_bwd_tc_workspace_bytes(batch, tokens, heads);
+}
+
+extern "C" int vdk_attention_bwd_tc(const void* qkv, const void* out, const void* d_out, const float* lse2, int batch, int tokens,
+                                    int heads, int head_dim, void* dqkv, void* workspace, size_t workspace_bytes, void* stream) {
+  VDK_REQUIRE(qkv && out && d_out && lse2 && dqkv, "vdk_attention_bwd_tc: null operand");
+  return launch_attention_bwd_pair(reinterpret_cast<const __nv_bfloat16*>(qkv), reinterpret_cast<const __nv_bfloat16*>(out),
+                                   reinterpret_cast<const __nv_bfloat16*>(d_out), lse2, batch, tokens, heads, head_dim,
+                                   reinterpret_cast<__nv_bfloat16*>(dqkv), workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int vdk_vit_forward(const vdk_vit_net* net, const float* images, int batch, int l2_normalize, float* embeddings,
@@ -723,6 +752,7 @@ struct VitTrainLayout {
   size_t xo[VDK_VIT_MAX_BLOCKS];                     // block outputs (residual stream)
   size_t f1, rf1, f2, rf2, z, zslab, bn_mean, bn_rstd;
   size_t dxa, dxb, dy, dbig, dz, dzb, gw, wslab, tok, dtok;
+  size_t att_d;                                      // D = rowsum(dO * O) [batch, heads, T] of the tcgen05 attention backward
   size_t total;
 };
 
@@ -731,7 +761,6 @@ static int vit_train_layout(const vdk_vit_net* n, int batch, VitTrainLayout* L) 
   int rc = vit_layout(n, batch, &base);
   if (rc != VDK_OK) return rc;
   VDK_REQUIRE(base.Kp == 3 * n->patch * n->patch, "vdk_vit_train: 3*patch*patch must be a multiple of 8 (patch %d)", n->patch);
-  VDK_REQUIRE(base.T <= kAttBwdMaxRows, "vdk_vit_train: at most %d tokens (got %d)", kAttBwdMaxRows, base.T);
   VDK_REQUIRE(batch > 1, "vdk_vit_train: batch must be > 1 (BatchNorm1d batch statistics)");
   L->N = base.N; L->T = base.T; L->C = base.C; L->Kp = base.Kp; L->M = base.M; L->depth = n->depth;
   const size_t M = L->M, C = L->C, F = n->feat_dim;
@@ -761,6 +790,7 @@ static int vit_train_layout(const vdk_vit_net* n, int batch, VitTrainLayout* L) 
   L->dz = take(static_cast<size_t>(batch) * F * 4); L->dzb = take(static_cast<size_t>(batch) * F * 2);
   L->gw = take(F * static_cast<size_t>(L->T) * C * 4);
   L->dtok = take(static_cast<size_t>(batch) * L->N * C * 2);
+  L->att_d = take(static_cast<size_t>(batch) * n->heads * L->T * 4);
   size_t slab = wgrad_slab_bytes(static_cast<int>(C), L->Kp, static_cast<size_t>(batch) * L->N);
   slab = std::max(slab, wgrad_slab_bytes(static_cast<int>(3 * C), static_cast<int>(C), M));
   slab = std::max(slab, wgrad_slab_bytes(static_cast<int>(C), static_cast<int>(C), M));
@@ -959,7 +989,12 @@ static int vit_backward_range(const vdk_vit_net* net, const vdk_vit_tensors* p, 
     RC(launch_col_sum(B16(dx), M, C, C, gb->proj_b, s));
     RC(G.wgrad(B16(dx), B16(L.att[i]), gb->proj_w, C, C, M, C, C, slabs, true));
     RC(G.run(B16(dx), b->proj_w, B16(L.dy), M, C, C, C, C, C, VDK_EPI_NONE, nullptr, nullptr, nullptr, 0, VDK_DTYPE_BF16, 1, 0, 0, 1));
-    RC(launch_attention_bwd(B16(L.qkv[i]), B16(L.att[i]), B16(L.dy), F32(L.lse[i]), batch, T, net->heads, kAttD, B16(L.dbig), s));
+    // up to 208 tokens (ViT-*/16 at 224^2) the mma.sync kernel that holds a head's whole P in shared memory; beyond, the tcgen05 pair
+    if (T <= kAttBwdMaxRows)
+      RC(launch_attention_bwd(B16(L.qkv[i]), B16(L.att[i]), B16(L.dy), F32(L.lse[i]), batch, T, net->heads, kAttD, B16(L.dbig), s));
+    else
+      RC(launch_attention_bwd_pair(B16(L.qkv[i]), B16(L.att[i]), B16(L.dy), F32(L.lse[i]), batch, T, net->heads, kAttD, B16(L.dbig),
+                                   ws + L.att_d, up256v(static_cast<size_t>(batch) * net->heads * T * 4), s));
     RC(launch_col_sum(B16(L.dbig), M, 3 * C, 3 * C, gb->qkv_b, s));
     RC(G.wgrad(B16(L.dbig), B16(L.y1[i]), gb->qkv_w, 3 * C, C, M, 3 * C, C, slabs, true));
     RC(G.run(B16(L.dbig), b->qkv_w, B16(L.dy), M, C, 3 * C, 3 * C, C, C, VDK_EPI_NONE, nullptr, nullptr, nullptr, 0, VDK_DTYPE_BF16, 1, 0, 0, 1));

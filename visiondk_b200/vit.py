@@ -6,7 +6,8 @@ timm 0.9.16's VisionTransformer (`model.patch_embed.proj`, `model.cls_token`, `m
 attn.qkv, attn.proj, norm2, mlp.fc1, mlp.fc2}`, `model.norm`) and `output_layer.{0: LayerNorm, 2: Linear, 3: BatchNorm1d}`,
 so reference checkpoints load with `strict=True`.  The eval forward runs in `vdk_vit_forward`, the train-mode forward and
 backward (BASELINE config 3) in `vdk_vit_train_forward` / `vdk_vit_train_backward` (csrc/vit.cu) as ONE autograd node;
-training needs 3*patch^2 % 8 == 0 and at most 208 tokens (ViT-*/16 at 224^2).
+training needs 3*patch^2 % 8 == 0 and takes any token count: the attention backward runs the mma.sync kernel up to 208 tokens
+(ViT-*/16 at 224^2) and the tcgen05 pair of csrc/attention_bwd_tc.cu beyond (ViT-*/8 at 224^2: 785 tokens; ViT-*/16 at 384^2: 577).
 """
 from __future__ import annotations
 
@@ -24,6 +25,11 @@ VIT_ARCHS = {
     "vit_small_patch16_224": (16, 384, 12, 6),
     "vit_base_patch16_224": (16, 768, 12, 12),
     "vit_large_patch16_224": (16, 1024, 24, 16),
+    "vit_small_patch8_224": (8, 384, 12, 6),
+    "vit_base_patch8_224": (8, 768, 12, 12),
+    "vit_small_patch16_384": (16, 384, 12, 6),
+    "vit_base_patch16_384": (16, 768, 12, 12),
+    "vit_large_patch16_384": (16, 1024, 24, 16),
     "vit_base_patch16_clip_224": (16, 768, 12, 12),
     "vit_large_patch14_clip_224": (14, 1024, 24, 16),
     "vit_large_patch14_clip_336": (14, 1024, 24, 16),
